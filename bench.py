@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline measurement of the event -> voxel-grid hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one voxel-grid build over one batch of synthetic events:
   N=1 : BASELINE.json configs[1] -- 50 M uniform events -> 5-bin 640x480 grid, reference
@@ -11,9 +11,10 @@ A "step" is one voxel-grid build over one batch of synthetic events:
 `value` is whole-job Mevents/s with the events resident in HBM, timed with CUDA events over
 exactly K steps, max over ranks.  `e2e` is the same metric through the public python API with
 pinned HOST tensors in and a host tensor out (H2D + D2H inside the timed region).
-`--impl reference` times the reference's OWN events_to_voxel_torch (the unmodified lib/ package that
-__graft_entry__.build() copies to the git-ignored baseline/_ref/, loaded through oracle/ref_loader.py) on the
-host cores; where that copy is missing it falls back to the library-op port (oracle/ref_port.py) and says so.
+`--impl reference` times the library-op port of the reference's events_to_voxel_torch (oracle/ref_port.py)
+on the host cores.
+`--dump-outputs DIR` writes the grid of the last timed step to DIR/voxel.npy (float32, B x H x W); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 Prints ONE JSON line on rank 0.
 """
 import argparse
@@ -181,19 +182,8 @@ def thread_candidates():
 
 
 def reference_functions():
-    """(kind, voxel_torch(xs,ys,ts,ps) -> grid, voxel_numpy(xs_int,ys_int,ts,ps) -> grid): the reference's own
-    events_to_voxel_torch / events_to_voxel (kind "reference", the unmodified lib/ copy in baseline/_ref/), or the
-    library-op port (kind "port") where that copy is not present."""
-    try:
-        from oracle import ref_loader
-        if ref_loader.available():
-            ref = ref_loader.load()
-            return ("reference",
-                    lambda xs, ys, ts, ps: ref.voxel_grid.events_to_voxel_torch(xs, ys, ts, ps, B, sensor_size=(H, W)),
-                    lambda xs, ys, ts, ps: ref.voxel_grid.events_to_voxel(xs, ys, ts, ps, B, sensor_size=(H, W)),
-                    ref_loader.REF_ROOT)
-    except Exception as exc:       # a broken copy must not cost the line: fall back and say so
-        print("bench: reference package unusable (%r), timing the library-op port" % (exc,), file=sys.stderr)
+    """(kind, voxel_torch(xs,ys,ts,ps) -> grid, voxel_numpy(xs_int,ys_int,ts,ps) -> grid): the library-op port of the
+    reference's events_to_voxel_torch / events_to_voxel."""
     from oracle import ref_port
     return ("port", lambda xs, ys, ts, ps: ref_port.voxel_torch_cpu(xs, ys, ts, ps, B, (H, W)),
             lambda xs, ys, ts, ps: ref_port.voxel_numpy(xs, ys, ts, ps, B, (H, W)), "oracle/ref_port.py")
@@ -234,7 +224,7 @@ def cpu_model():
 
 
 def run_reference(args, rank, world):
-    """--impl reference: the reference's own CPU path on the host cores (see reference_functions)."""
+    """--impl reference: the port of the reference's CPU path on the host cores (see reference_functions)."""
     if rank != 0:
         return
     kind, voxel_torch, _, where = reference_functions()
@@ -257,11 +247,12 @@ def run_reference(args, rank, world):
         voxel_torch(xs, ys, ts, ps)
     s = time.perf_counter()
     for _ in range(args.steps):
-        voxel_torch(xs, ys, ts, ps)
+        res = voxel_torch(xs, ys, ts, ps)
     el = time.perf_counter() - s
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, voxel=res)
     value = n * args.steps / el / 1e6
-    what = ("the reference's own events_to_voxel_torch (unmodified lib/ package from %s)" % where if kind == "reference" else
-            "events_to_voxel_torch library-op port (oracle/ref_port.py; the reference package is not present here)")
+    what = "events_to_voxel_torch library-op port (%s)" % where
     sample = ("%s, torch CPU f32, %d threads = the fastest of %s on this host; %s per step" % (
         what, torch.get_num_threads(), thread_candidates(),
         "the FULL 50M-event workload" if n == N_PER_GPU else
@@ -378,6 +369,8 @@ def run_ours(args, rank, local_rank, world):
     else:
         expect = float(p.double().sum())
     assert abs(total - expect) <= 1e-6 * n * world + 4.0, (total, expect)
+    if args.dump_outputs and rank == 0:        # every rank holds the same reduced grid
+        dump_outputs(args.dump_outputs, voxel=out)
 
     value = n * world * args.steps / elapsed_ms / 1e3          # Mevents/s, whole job
     peak, peak_src = measured_peak()
@@ -499,10 +492,9 @@ def run_ours(args, rank, local_rank, world):
         best = max(cpu_t["torch_cpu_mevs"], cpu_t["numpy_mevs"])
         used = cpu_t["torch_threads"] if cpu_t["torch_cpu_mevs"] >= cpu_t["numpy_mevs"] else 1
         cpu = {"value": best, "unit": "Mevents/s", "cores": used, "host_cores": cpu_t["cores"], "kind": cpu_t["kind"],
-               "sample": "%d-event sample of the workload, best of 3; faster of the %s events_to_voxel_torch on torch-CPU "
-                         "(%.1f Mev/s, %d threads) and events_to_voxel on numpy (%.1f Mev/s, 1 thread); from %s"
-                         % (CPU_SAMPLE, "reference's own" if cpu_t["kind"] == "reference" else "library-op port of",
-                            cpu_t["torch_cpu_mevs"], cpu_t["torch_threads"], cpu_t["numpy_mevs"], cpu_t["where"]),
+               "sample": "%d-event sample of the workload, best of 3; faster of the library-op port of events_to_voxel_torch "
+                         "on torch-CPU (%.1f Mev/s, %d threads) and events_to_voxel on numpy (%.1f Mev/s, 1 thread); from %s"
+                         % (CPU_SAMPLE, cpu_t["torch_cpu_mevs"], cpu_t["torch_threads"], cpu_t["numpy_mevs"], cpu_t["where"]),
                "cpu": cpu_model()}
         if not args.no_extra:
             del x, y, t, p
@@ -863,6 +855,13 @@ def secondary_metrics(L, _lib, device, peak):
     return out
 
 
+def dump_outputs(directory, **arrays):
+    """Write each array as DIR/<name>.npy in float32."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a.detach().to("cpu", torch.float32).numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -870,6 +869,7 @@ def main():
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary (cmax) numbers")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the grid of the last timed step to DIR/voxel.npy")
     args = ap.parse_args()
     rank, world, local_rank = env_int("RANK", 0), env_int("WORLD_SIZE", 1), env_int("LOCAL_RANK", 0)
     if args.impl == "reference":

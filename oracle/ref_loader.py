@@ -1,11 +1,8 @@
 """Loader for the UNMODIFIED reference (TimoStoff/event_utils) -- TEST / BASELINE INFRASTRUCTURE ONLY.
 
-Where the reference lives: ``$EVK_REFERENCE_ROOT``, else ``/root/reference`` (the build container), else the
-unmodified copy of its ``lib/`` package that ``__graft_entry__.build()`` places in the git-ignored
-``baseline/_ref/`` (which travels to the GPU box with the gpurun snapshot; /root/reference does not).
-It is used by ``tests/golden/make_golden.py`` to generate the committed golden vectors, by the ``not gpu``
-tests that pin the oracle restatement against the real reference, by ``bench.py --impl reference`` /
-``cpu_baseline`` (the reference's own functions timed on the host cores) and by the module-swap tests.
+Where the reference lives: ``$EVK_REFERENCE_ROOT`` (a checkout of TimoStoff/event_utils).  It is used by
+``tests/golden/make_golden.py`` and ``tests/golden/make_reference_checks.py`` to generate the committed golden
+vectors and by the module-swap test, which runs the reference's own callers and skips where it is absent.
 
 Two of the hot-path files do not parse as shipped (SURVEY.md section 8c):
   * lib/contrast_max/warps.py:7-10  class docstring at column 0, :81 stray text, :3 bogus import
@@ -19,23 +16,12 @@ import os
 import sys
 import types
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
 
-
-def _find_root():
-    cands = [os.environ.get("EVK_REFERENCE_ROOT"), "/root/reference",
-             os.path.join(os.path.dirname(_HERE), "baseline", "_ref")]
-    for c in cands:
-        if c and os.path.isdir(os.path.join(c, "lib", "representations")):
-            return c
-    return cands[0] or cands[1]
-
-
-REF_ROOT = _find_root()
+REF_ROOT = os.environ.get("EVK_REFERENCE_ROOT", "")
 
 
 def available():
-    return os.path.isdir(os.path.join(REF_ROOT, "lib", "representations"))
+    return bool(REF_ROOT) and os.path.isdir(os.path.join(REF_ROOT, "lib", "representations"))
 
 
 def _stub(name, **attrs):

@@ -1,9 +1,9 @@
 """Generate the golden vectors in tests/golden/ by running the UNMODIFIED reference
-(/root/reference, loaded through oracle/ref_loader.py).  Run in the build container only:
+(loaded through oracle/ref_loader.py):
 
-    python tests/golden/make_golden.py
+    EVK_REFERENCE_ROOT=<checkout of TimoStoff/event_utils> python tests/golden/make_golden.py
 
-The .npz files are committed; the GPU box (which has no /root/reference) only reads them.
+The .npz files are committed; the tests only read them.
 Every case stores its inputs and the reference's outputs.
 """
 import os
@@ -14,6 +14,8 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import cmax_scenes  # noqa: E402
 from oracle import ref_loader  # noqa: E402
 
 OUT = os.path.dirname(os.path.abspath(__file__))
@@ -228,12 +230,11 @@ scenes = {
     "c9": events(0, 20000, 180, 240),  # SURVEY Appendix C9 draw order is reproduced below
     "lat": lattice(7, 30000),
 }
-rng = np.random.default_rng(0)
-N = 20000
-scenes["c9"] = (rng.random(N) * 239, rng.random(N) * 179, np.sort(rng.random(N)) * 0.1, rng.integers(0, 2, N) * 2.0 - 1)
+scenes["c9"] = cmax_scenes.c9_events()
+cases["c9_sha256"] = np.array(cmax_scenes.c9_sha256(scenes["c9"]))     # regenerated by the tests, not stored
+cases.update({"lat" + k: a for k, a in zip(("_x", "_y", "_t", "_p"), scenes["lat"])})
 evals = []
 for sname, (xs, ys, ts, ps) in scenes.items():
-    cases.update({sname + "_x": xs, sname + "_y": ys, sname + "_t": ts, sname + "_p": ps})
     for params in [(30.0, -20.0), (60.0, -35.0), (45.0, -20.0), (0.0, 0.0)]:
         for sigma in (1.0, 0.0, 2.3):
             f = obj.evaluate_function(params, xs, ys, ts, ps, warp, (180, 240), sigma)

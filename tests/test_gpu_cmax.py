@@ -4,6 +4,7 @@ import copy
 import numpy as np
 import pytest
 
+import cmax_scenes
 from conftest import assert_close_to_max, golden, make_events
 
 pytestmark = pytest.mark.gpu
@@ -33,7 +34,7 @@ def test_golden_f_and_g():
     for row in g["evals"]:
         s, vx, vy, sigma, f_ref, g0, g1 = row
         tag = scenes[int(s)]
-        ev = [g[tag + k] for k in ("_x", "_y", "_t", "_p")]
+        ev = cmax_scenes.events(g, tag)
         f = obj.evaluate_function((vx, vy), *ev, warp, (180, 240), sigma)
         gr = obj.evaluate_gradient((vx, vy), *ev, warp, (180, 240), sigma)
         assert isinstance(f, float) and isinstance(gr, np.ndarray) and gr.shape == (2,)
@@ -82,7 +83,7 @@ def test_get_iwe_and_precomputed_forms():
     gp = obj.evaluate_gradient(iwe=g["lat_iwe"], d_iwe=g["lat_diwe"], blur_sigma=1.0)
     assert np.abs(gp - g["pre_g"]).max() <= 1e-5 * np.abs(g["pre_g"]).max()
     # img_size larger than the fixed 180x240 sensor (quirk B7)
-    c9 = [g["c9" + k] for k in ("_x", "_y", "_t", "_p")]
+    c9 = cmax_scenes.events(g, "c9")
     fb = obj.evaluate_function((30.0, -20.0), c9[0] * 2, c9[1] * 2, c9[2], c9[3], warp, (480, 640), 1.0)
     assert abs(fb - g["c9_f_big"]) <= 1e-5 * abs(g["c9_f_big"])
 

@@ -1,8 +1,8 @@
 """The reference's OWN callers on top of this repo's kernels (VERDICT r1 weak #6): the `sys.modules` aliasing that
 INTEGRATION.md section 1 advertises, then the unmodified `optimize_contrast` (lib/contrast_max/events_cmax.py:313-346) and
-`BaseVoxelDataset.get_voxel_grid` (lib/data_loaders/base_dataset.py:433-455) from the reference package
-(/root/reference in the build container, the unmodified copy in baseline/_ref on the GPU box).  Runs in a subprocess so
-that the aliased modules do not leak into the other tests."""
+`BaseVoxelDataset.get_voxel_grid` (lib/data_loaders/base_dataset.py:433-455) from the reference package at
+$EVK_REFERENCE_ROOT; the repository cannot hold that package's source, so the test skips where it is absent.
+Runs in a subprocess so that the aliased modules do not leak into the other tests."""
 import os
 import subprocess
 import sys
@@ -80,7 +80,7 @@ print("get_voxel_grid ok")
 def test_reference_callers_run_on_the_swapped_modules():
     from oracle import ref_loader
     if not ref_loader.available():
-        pytest.skip("reference package present neither at /root/reference nor in baseline/_ref")
+        pytest.skip("reference package not found (set EVK_REFERENCE_ROOT)")
     out = subprocess.run([sys.executable, "-c", SCRIPT % {"root": ROOT}], capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-4000:]
     assert "get_voxel_grid ok" in out.stdout

@@ -3,6 +3,7 @@ reference (tests/golden/make_golden.py).  Runs without a GPU.  This is the oracl
 import numpy as np
 import pytest
 
+import cmax_scenes
 from conftest import assert_close_to_max, golden
 
 
@@ -123,8 +124,7 @@ def test_cmax_f_and_g(oracle):
     for row in g["evals"]:
         s, vx, vy, sigma, f_ref, g0, g1 = row
         tag = scenes[int(s)]
-        f, grad = oracle.cmax_variance((vx, vy), g[tag + "_x"], g[tag + "_y"], g[tag + "_t"], g[tag + "_p"],
-                                       blur_sigma=sigma)
+        f, grad = oracle.cmax_variance((vx, vy), *cmax_scenes.events(g, tag), blur_sigma=sigma)
         assert abs(f - f_ref) <= 1e-6 * abs(f_ref) + 1e-12, (tag, vx, vy, sigma, f, f_ref)
         gref = np.array([g0, g1])
         assert np.abs(grad - gref).max() <= 2e-5 * np.abs(gref).max() + 1e-9, (tag, vx, vy, sigma, grad, gref)
