@@ -37,6 +37,8 @@ CMAX_WANT_GRAD = 0x10
 CMAX_ABS_POLARITY = 0x20
 CMAX_NO_CHANNEL_MIX = 0x40
 OBJ_VARIANCE, OBJ_SOS, OBJ_SOE, OBJ_MOA, OBJ_ISOA, OBJ_SOSA = range(6)
+WARP_LINVEL, WARP_ROTATION, WARP_XYZTHETA = range(3)
+WARP_MODELS = {"linvel": WARP_LINVEL, "rotation": WARP_ROTATION, "xyztheta": WARP_XYZTHETA}   # warp_function.fused_kind
 
 _lib = None
 _lock = threading.Lock()
@@ -111,6 +113,16 @@ def _declare(L):
                                                       vp, vp, sz, vp]
     L.evk_iwe_objective_f32.restype = ci
     L.evk_iwe_objective_f32.argtypes = [vp, vp, ci, ci, f64, cu, ci, f64, vp, vp, sz, vp]
+    L.evk_cmax_model_objective_f64.restype = ci
+    L.evk_cmax_model_objective_f64.argtypes = [ci, vp, ci, vp, vp, vp, vp, i64, f64, f64, ci, ci, ci, ci, f64, cu, ci, f64,
+                                               vp, vp, vp, sz, vp]
+    L.evk_cmax_model_objective_f32.restype = ci
+    L.evk_cmax_model_objective_f32.argtypes = [ci, vp, ci, vp, vp, vp, vp, i64, f32, ci, ci, ci, ci, f64, cu, ci, f64,
+                                               vp, vp, vp, sz, vp]
+    L.evk_cmax_model_warp_f64.restype = ci
+    L.evk_cmax_model_warp_f64.argtypes = [ci, vp, ci, vp, vp, vp, vp, i64, f64, ci, ci, cu, vp, vp, vp, vp, vp, vp]
+    L.evk_iwe_objective_k_f32.restype = ci
+    L.evk_iwe_objective_k_f32.argtypes = [vp, vp, ci, ci, ci, f64, cu, ci, f64, vp, vp, vp, sz, vp]
     L.evk_gaussian_blur_f32.restype = ci
     L.evk_gaussian_blur_f32.argtypes = [vp, ci, ci, f64, vp, vp, vp]
     L.evk_variance_objective_f32.restype = ci

@@ -12,7 +12,7 @@ import numpy as np
 import scipy.optimize as opt
 
 from ..util.event_util import infer_resolution
-from .objectives import evaluate_candidates, get_iwe, pinned_events, soe_objective, variance_objective
+from .objectives import _fused_kind, evaluate_candidates, get_iwe, pinned_events, soe_objective, variance_objective
 from .warps import linvel_warp
 
 
@@ -58,20 +58,21 @@ def optimize_contrast(xs, ys, ts, ps, warp_function, objective, optimizer=opt.fm
     """
     Gradient-based contrast maximisation; same signature as events_cmax.py:313-346.  With
     grid_search_init the start point comes from grid_search_initial (the reference calls an
-    undefined `recursive_search` there, events_cmax.py:336).
+    undefined `recursive_search` there, events_cmax.py:336).  The default start point is zeros(warp_function.dims)
+    (the reference's [0, 0] only fits 2-parameter models).
     @returns the maximising warp parameters
     """
     # nothing between here and the return modifies the event arrays (scipy hands the same `args` objects to
     # every f / f' call), so the event set is uploaded and hashed ONCE for the whole optimisation
-    fused = getattr(warp_function, "fused_kind", None) == "linvel"
+    fused = _fused_kind(warp_function) is not None
     with (pinned_events(xs, ys, ts, ps) if fused else contextlib.nullcontext()):
         if grid_search_init and x0 is None:
             init_obj = copy.deepcopy(objective)
             init_obj.adaptive_lifespan = False
             x0 = grid_search_initial(xs, ys, ts, ps, warp_function, init_obj, img_size, log_scale=False)["min_params"]
-            x0 = np.array([0, 0]) if x0 is None else np.array(x0)
+            x0 = np.zeros(warp_function.dims) if x0 is None else np.array(x0)
         elif x0 is None:
-            x0 = np.array([0, 0])
+            x0 = np.zeros(warp_function.dims)
         objective.iter_update(x0)
         args = (xs, ys, ts, ps, warp_function, img_size, blur_sigma)
         if numeric_grads:

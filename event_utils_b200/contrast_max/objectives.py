@@ -7,7 +7,8 @@ The reference rebuilds everything from the raw host arrays for every f and every
   * the event arrays are uploaded to the GPU once and cached (the optimiser hands over the same
     numpy arrays at every iteration, events_cmax.py:341);
   * warp + bounds mask + IWE + derivative images + blur + variance + gradient is ONE fused
-    evaluation (csrc/evk_cmax.cu) that returns f and g together;
+    evaluation (csrc/evk_cmax.cu) that returns f and g together -- for linvel_warp, pure_rotation_warp and
+    xyztheta_warp (warps.py, `fused_kind`); the last two take a second pass over the events for g;
   * (params -> f, g) is memoised, so scipy's separate f / f' calls at the same point cost one
     launch.
 Objects keep the reference's attributes and calling conventions (positional `args=` form,
@@ -119,11 +120,12 @@ def _result_buffers(dev):
     last kernel of an evaluation writes straight over PCIe (pinned allocations are device-addressable
     under unified addressing), so reading a result back is one stream synchronise -- no device buffer,
     no D2H copy operation (a fresh torch.zeros + pageable .cpu() per call cost ~25 us of a ~90 us
-    evaluation, a pinned mirror + copy_ still ~10 us).  Returns (tensor, numpy view)."""
+    evaluation, a pinned mirror + copy_ still ~10 us).  Slots 0..11 hold the result, 12..19 the gradient of a model with up to 8 parameters.
+    Returns (tensor, numpy view)."""
     k = (dev, torch.cuda.current_stream(dev).cuda_stream, threading.get_ident())   # per stream AND host thread: reuse is only safe in stream order
     b = _result_bufs.get(k)
     if b is None:
-        host = torch.zeros(12, dtype=torch.float64).pin_memory()
+        host = torch.zeros(20, dtype=torch.float64).pin_memory()
         b = (host, host.numpy())
         _result_bufs[k] = b
     return b
@@ -146,11 +148,17 @@ class _on_device:
             self.ctx.__exit__(*exc)
 
 
-def _fused_linvel(params, xs, ys, ts, ps, img_size, blur_sigma, want_grad, use_polarity,
-                  first=0, last=None, p_scale=1.0, want_images=False, channel_mix=True,
-                  objective=_lib.OBJ_VARIANCE, obj_param=0.0, ev=None):
-    """One fused evaluation on events [first:last) of the cached device copy.
-    Returns (result[8] as numpy f64, iwe or None, d_iwe or None)."""
+def _fused_kind(warpfunc):
+    """The model the fused kernels evaluate for this warp object ("linvel", "rotation", "xyztheta"), or None."""
+    kind = getattr(warpfunc, "fused_kind", None)
+    return kind if kind in _lib.WARP_MODELS else None
+
+
+def _fused_eval(params, xs, ys, ts, ps, img_size, blur_sigma, want_grad, use_polarity,
+                first=0, last=None, p_scale=1.0, want_images=False, channel_mix=True,
+                objective=_lib.OBJ_VARIANCE, obj_param=0.0, ev=None, kind="linvel"):
+    """One fused evaluation of motion model `kind` on events [first:last) of the cached device copy.
+    Returns (result[12] as numpy f64, gradient[dims], iwe or None, d_iwe or None); the images are linvel's only."""
     L = _lib.lib()
     ev = _device_events(xs, ys, ts, ps) if ev is None else ev
     n_all = ev.n
@@ -173,6 +181,35 @@ def _fused_linvel(params, xs, ys, ts, ps, img_size, blur_sigma, want_grad, use_p
             | {None: 0, "onchip": _lib.VARIANT_SMEM_TILE, "l2": _lib.VARIANT_VECTOR_RED}[event_pass]
         sigma = float(blur_sigma) if blur_sigma is not None else 0.0
         # the reference warps to the LAST timestamp of the (possibly sliced) event set (objectives.py:186)
+        if kind != "linvel":
+            dims = {"rotation": 3, "xyztheta": 4}[kind]
+            prm = np.ascontiguousarray(np.asarray(params, dtype=np.float64).reshape(-1))
+            if prm.shape[0] != dims:
+                raise ValueError("the %s model takes %d parameters, %d given" % (kind, dims, prm.shape[0]))
+            grad_ptr = result.data_ptr() + 12 * 8
+            if ev.mode == "f64":
+                t_ref = float(ev.t[last - 1].item()) if last != n_all else ev.t_last
+                off = first * 8
+                _lib.check(L.evk_cmax_model_objective_f64(
+                    _lib.WARP_MODELS[kind], prm.ctypes.data, dims, ev.x.data_ptr() + off, ev.y.data_ptr() + off,
+                    ev.t.data_ptr() + off, ev.p.data_ptr() + off, n, float(p_scale), t_ref, int(img_size[0]), int(img_size[1]),
+                    Hs, Ws, sigma, flags, int(objective), float(obj_param), _lib.ptr(result), grad_ptr, _lib.ptr(ws), ws.numel(),
+                    _lib.stream()))
+            else:
+                if last != n_all:
+                    raise NotImplementedError("f32 fast mode stores t relative to the last event; "
+                                              "slicing the tail (adaptive_lifespan) needs precision='f64'")
+                off = first * 4
+                _lib.check(L.evk_cmax_model_objective_f32(
+                    _lib.WARP_MODELS[kind], prm.ctypes.data, dims, ev.x.data_ptr() + off, ev.y.data_ptr() + off,
+                    ev.t.data_ptr() + off, ev.p.data_ptr() + off, n, float(p_scale), int(img_size[0]), int(img_size[1]),
+                    Hs, Ws, sigma, flags, int(objective), float(obj_param), _lib.ptr(result), grad_ptr, _lib.ptr(ws), ws.numel(),
+                    _lib.stream()))
+            torch.cuda.current_stream().synchronize()
+            res, grad = result_view[:12].copy(), result_view[12:12 + dims].copy()
+            if res[4] != 0:
+                raise IndexError("%d warped events index outside the IWE canvas %s" % (int(res[4]), (Hs + 1, Ws + 1)))
+            return res, (grad if want_grad else np.zeros(dims)), None, None
         if ev.mode == "f64":
             t_ref = float(ev.t[last - 1].item()) if last != n_all else ev.t_last
             off = first * 8
@@ -192,27 +229,69 @@ def _fused_linvel(params, xs, ys, ts, ps, img_size, blur_sigma, want_grad, use_p
                 Hs, Ws, sigma, flags, int(objective), float(obj_param), _lib.ptr(result), _lib.ptr(iwe), _lib.ptr(d_iwe),
                 _lib.ptr(ws), ws.numel(), _lib.stream()))
         torch.cuda.current_stream().synchronize()
-        res = result_view.copy()
+        res = result_view[:12].copy()
         if res[4] != 0:
             raise IndexError("%d warped events index outside the IWE canvas %s" % (int(res[4]), (Hs + 1, Ws + 1)))
-        return res, (iwe.cpu().numpy() if iwe is not None else None), (d_iwe.cpu().numpy() if d_iwe is not None else None)
+        return res, res[1:3].copy(), (iwe.cpu().numpy() if iwe is not None else None), \
+            (d_iwe.cpu().numpy() if d_iwe is not None else None)
+
+
+def _model_images(kind, params, xs, ys, ts, ps, img_size, compute_gradient, use_polarity):
+    """get_iwe for the rotation / xyztheta models: warp, mask and Jacobians on the device
+    (evk_cmax_model_warp_f64), then the image and its `dims` derivative images (evk_image_drv_f32)."""
+    L = _lib.lib()
+    dims = {"rotation": 3, "xyztheta": 4}[kind]
+    prm = np.ascontiguousarray(np.asarray(params, dtype=np.float64).reshape(-1))
+    if prm.shape[0] != dims:
+        raise ValueError("the %s model takes %d parameters, %d given" % (kind, dims, prm.shape[0]))
+    if precision == "f64":
+        ev = _device_events(xs, ys, ts, ps)
+        x, y, t, p, n, t_ref = ev.x, ev.y, ev.t, ev.p, ev.n, ev.t_last
+    else:
+        # the warp is f64 whatever the fast mode of the objective stores
+        host = [np.ascontiguousarray(np.asarray(a, dtype=np.float64).reshape(-1)) for a in (xs, ys, ts, ps)]
+        x, y, t, p = _lib.upload([torch.from_numpy(a) for a in host], E.compute_device())
+        n, t_ref = host[0].shape[0], float(host[2][-1]) if host[2].shape[0] else 0.0
+    if n == 0:
+        raise IndexError("index -1 is out of bounds for axis 0 with size 0")
+    Hs, Ws = SENSOR_SIZE
+    dev = x.device
+    with _on_device(dev):
+        xw, yw, pw = (torch.empty(n, dtype=torch.float32, device=dev) for _ in range(3))
+        jx = torch.empty((dims, n), dtype=torch.float32, device=dev) if compute_gradient else None
+        jy = torch.empty((dims, n), dtype=torch.float32, device=dev) if compute_gradient else None
+        _lib.check(L.evk_cmax_model_warp_f64(
+            _lib.WARP_MODELS[kind], prm.ctypes.data, dims, x.data_ptr(), y.data_ptr(), t.data_ptr(), p.data_ptr(), n, t_ref,
+            int(img_size[0]), int(img_size[1]), 0 if use_polarity else _lib.CMAX_ABS_POLARITY, _lib.ptr(xw), _lib.ptr(yw),
+            _lib.ptr(pw), _lib.ptr(jx), _lib.ptr(jy), _lib.stream()))
+        img = torch.empty((Hs + 1, Ws + 1), dtype=torch.float32, device=dev)
+        d_img = torch.empty((dims, Hs + 1, Ws + 1), dtype=torch.float32, device=dev) if compute_gradient else None
+        oob = _lib.oob_counter(dev)
+        _lib.check(L.evk_image_drv_f32(_lib.ptr(xw), _lib.ptr(yw), _lib.ptr(pw), _lib.ptr(jx), _lib.ptr(jy),
+                                       dims if compute_gradient else 0, n, Hs + 1, Ws + 1, float(Ws), float(Hs), _lib.CLIP,
+                                       _lib.ptr(img), _lib.ptr(d_img), _lib.ptr(oob), _lib.stream()))
+        E.raise_if_oob(oob, "image", (Hs + 1, Ws + 1))
+        return img.cpu().numpy(), (d_img.cpu().numpy() if d_img is not None else None)
 
 
 def _objective_of_images(iwe, d_iwe, blur_sigma, want_grad, objective=_lib.OBJ_VARIANCE, obj_param=0.0):
-    """objective (+ gradient) of precomputed images, on the GPU (evk_iwe_objective_f32)."""
+    """objective (+ gradient) of precomputed images with any number K <= 8 of derivative channels, on the GPU
+    (evk_iwe_objective_k_f32).  Returns (result[12], gradient[K] or None)."""
     L = _lib.lib()
     dev = E.compute_device()
     iwe = np.ascontiguousarray(iwe, dtype=np.float32)
     with torch.cuda.device(dev):
         a = torch.from_numpy(iwe).to(dev)
         d = torch.from_numpy(np.ascontiguousarray(d_iwe, dtype=np.float32)).to(dev) if d_iwe is not None else None
+        K = d.shape[0] if d is not None else 0
         ws = _lib.scratch("cmax_ws", L.evk_cmax_workspace_bytes(iwe.shape[0] - 1, iwe.shape[1] - 1), dev)
-        result = torch.zeros(12, dtype=torch.float64, device=dev)
+        result = torch.zeros(12 + max(K, 1), dtype=torch.float64, device=dev)
         flags = _lib.CMAX_WANT_GRAD if (want_grad and d is not None) else 0
-        _lib.check(L.evk_iwe_objective_f32(_lib.ptr(a), _lib.ptr(d), iwe.shape[0], iwe.shape[1], float(blur_sigma), flags,
-                                           int(objective), float(obj_param), _lib.ptr(result), _lib.ptr(ws), ws.numel(),
-                                           _lib.stream()))
-        return result.cpu().numpy()
+        _lib.check(L.evk_iwe_objective_k_f32(_lib.ptr(a), _lib.ptr(d), K, iwe.shape[0], iwe.shape[1], float(blur_sigma), flags,
+                                             int(objective), float(obj_param), _lib.ptr(result), result.data_ptr() + 12 * 8,
+                                             _lib.ptr(ws), ws.numel(), _lib.stream()))
+        out = result.cpu().numpy()
+        return out[:12], (out[12:12 + K] if K else None)
 
 
 # ---------------------------------------------------------------------------------------------
@@ -287,10 +366,12 @@ def get_iwe(params, xs, ys, ts, ps, warpfunc, img_size, compute_gradient=False,
     objectives.py:165-199.  numpy in, numpy float32 (181,241) / (dims,181,241) out.
     @returns tuple: iwe, d_iwe (or None) [, (xs_warped, ys_warped)] [, per-event contrast]
     """
-    fused = getattr(warpfunc, "fused_kind", None) == "linvel"
-    if fused and not return_events and not return_per_event_contrast:
-        _, iwe, d_iwe = _fused_linvel(params, xs, ys, ts, ps, img_size, 0.0, compute_gradient, use_polarity,
-                                      want_images=True)
+    kind = _fused_kind(warpfunc)
+    if kind is not None and not return_events and not return_per_event_contrast:
+        if kind != "linvel":
+            return _model_images(kind, params, xs, ys, ts, ps, img_size, compute_gradient, use_polarity)
+        _, _, iwe, d_iwe = _fused_eval(params, xs, ys, ts, ps, img_size, 0.0, compute_gradient, use_polarity,
+                                       want_images=True)
         return (iwe, d_iwe)
     # generic warp objects (and the two debugging outputs): host warp + mask as in the
     # reference, image formation on the GPU
@@ -333,22 +414,23 @@ class variance_objective(objective_function):
                 self.recompute_lifespan = False
             first, last, scale = int(self.s_idx), -1, 100.0   # xs[s_idx:-1], ps*100 (objectives.py:224-225)
         blur_sigma = self.default_blur if blur_sigma is None else blur_sigma
-        fused = getattr(warpfunc, "fused_kind", None) == "linvel"
+        kind = _fused_kind(warpfunc)
+        fused = kind is not None
         ev = _device_events(xs, ys, ts, ps) if fused else None
-        # memo only for the fused warp: a generic warp object's result depends on that object's identity and state
-        key = (tuple(float(v) for v in params), ev.key, tuple(img_size), float(blur_sigma), first, last, scale,
+        # memo only for the fused warps: a generic warp object's result depends on that object's identity and state
+        key = (kind, tuple(float(v) for v in params), ev.key, tuple(img_size), float(blur_sigma), first, last, scale,
                self.use_polarity, precision) if fused else None
         if fused and self._memo is not None and self._memo[0] == key:
             return self._memo[1], self._memo[2]
         if fused:
-            res, _, _ = _fused_linvel(params, xs, ys, ts, ps, img_size, blur_sigma, True, self.use_polarity,
-                                      first=first, last=last, p_scale=scale, ev=ev)
+            res, g, _, _ = _fused_eval(params, xs, ys, ts, ps, img_size, blur_sigma, True, self.use_polarity,
+                                       first=first, last=last, p_scale=scale, ev=ev, kind=kind)
         else:
             sl = slice(first, last)
             iwe, d_iwe = get_iwe(params, xs[sl], ys[sl], ts[sl], ps[sl] * scale, warpfunc, img_size,
                                  use_polarity=self.use_polarity, compute_gradient=True)
-            res = _objective_of_images(iwe, d_iwe, blur_sigma, True)
-        f, g = float(res[0]), np.array([res[1], res[2]])
+            res, g = _objective_of_images(iwe, d_iwe, blur_sigma, True)
+        f = float(res[0])
         self._memo = (key, f, g) if fused else None
         return f, g
 
@@ -357,7 +439,7 @@ class variance_objective(objective_function):
         """-var(blurred IWE) at `params` (or of a precomputed `iwe`)."""
         if iwe is not None:
             blur_sigma = self.default_blur if blur_sigma is None else blur_sigma
-            return float(_objective_of_images(iwe, None, blur_sigma, False)[0])
+            return float(_objective_of_images(iwe, None, blur_sigma, False)[0][0])
         f, _ = self._evaluate(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma)
         return f
 
@@ -366,8 +448,7 @@ class variance_objective(objective_function):
         """Analytic gradient of the objective wrt the warp parameters (np.ndarray[dims])."""
         if iwe is not None and d_iwe is not None:
             blur_sigma = self.default_blur if blur_sigma is None else blur_sigma
-            res = _objective_of_images(iwe, d_iwe, blur_sigma, True)
-            return np.array([res[1], res[2]])
+            return _objective_of_images(iwe, d_iwe, blur_sigma, True)[1]
         _, g = self._evaluate(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma)
         return g.copy()
 
@@ -385,29 +466,32 @@ class _fused_objective(objective_function):
         return 0.0
 
     def _result(self, params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=None, d_iwe=None, want_grad=True):
+        """(result[12], gradient[dims] or None) of one evaluation"""
         blur_sigma = self.default_blur if blur_sigma is None else blur_sigma
         if iwe is not None:
             return _objective_of_images(iwe, d_iwe, blur_sigma, want_grad and d_iwe is not None, self._kind, self._param())
-        fused = getattr(warpfunc, "fused_kind", None) == "linvel"
+        kind = _fused_kind(warpfunc)
+        fused = kind is not None
         ev = _device_events(xs, ys, ts, ps) if fused else None
-        key = (tuple(float(v) for v in params), ev.key, tuple(img_size), float(blur_sigma), self.use_polarity,
+        key = (kind, tuple(float(v) for v in params), ev.key, tuple(img_size), float(blur_sigma), self.use_polarity,
                precision, self._kind, self._param()) if fused else None
         memo = getattr(self, "_memo", None)
         if fused and memo is not None and memo[0] == key:
             return memo[1]
         if fused:
-            res, _, _ = _fused_linvel(params, xs, ys, ts, ps, img_size, blur_sigma, self.has_derivative, self.use_polarity,
-                                      objective=self._kind, obj_param=self._param(), ev=ev)
+            res, g, _, _ = _fused_eval(params, xs, ys, ts, ps, img_size, blur_sigma, self.has_derivative, self.use_polarity,
+                                       objective=self._kind, obj_param=self._param(), ev=ev, kind=kind)
+            out = (res, g)
         else:
             img, dimg = get_iwe(params, xs, ys, ts, ps, warpfunc, img_size, use_polarity=self.use_polarity,
                                 compute_gradient=self.has_derivative)
-            res = _objective_of_images(img, dimg, blur_sigma, self.has_derivative, self._kind, self._param())
-        self._memo = (key, res) if fused else None
-        return res
+            out = _objective_of_images(img, dimg, blur_sigma, self.has_derivative, self._kind, self._param())
+        self._memo = (key, out) if fused else None
+        return out
 
     def evaluate_function(self, params=None, xs=None, ys=None, ts=None, ps=None,
             warpfunc=None, img_size=None, blur_sigma=None, showimg=False, iwe=None):
-        return float(self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)[0])
+        return float(self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)[0][0])
 
     def evaluate_gradient(self, params=None, xs=None, ys=None, ts=None, ps=None,
             warpfunc=None, img_size=None, blur_sigma=None, showimg=False, iwe=None, d_iwe=None):
@@ -415,8 +499,8 @@ class _fused_objective(objective_function):
             return None
         if iwe is not None and d_iwe is None:
             iwe = None
-        res = self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, d_iwe=d_iwe)
-        return np.array([res[1], res[2]])
+        _, g = self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, d_iwe=d_iwe)
+        return np.array(g)
 
 
 class rms_objective(_fused_objective):
@@ -476,7 +560,7 @@ class moa_objective(_fused_objective):
 
     def evaluate_function(self, params=None, xs=None, ys=None, ts=None, ps=None,
             warpfunc=None, img_size=None, blur_sigma=None, showimg=False, iwe=None):
-        return float(self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)[0])
+        return float(self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)[0][0])
 
 
 class isoa_objective(_fused_objective):
@@ -519,7 +603,7 @@ class r1_objective(_fused_objective):
 
     def evaluate_function(self, params=None, xs=None, ys=None, ts=None, ps=None,
             warpfunc=None, img_size=None, blur_sigma=None, showimg=False, iwe=None):
-        res = self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)
+        res, _ = self._result(params, xs, ys, ts, ps, warpfunc, img_size, blur_sigma, iwe=iwe, want_grad=False)
         sos, sosa = float(res[8]), float(res[9])
         if sosa > self.last_sosa:
             return -sos

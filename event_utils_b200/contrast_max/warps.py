@@ -1,10 +1,10 @@
 """Motion models for contrast maximisation -- drop-in for the reference's lib/contrast_max/warps.py
 (`warp_function` ABC :6-42, `linvel_warp` :44-61, the two empty stubs :63-83).
 
-An objective from `event_utils_b200.contrast_max.objectives` that is handed a `linvel_warp` never
-calls `warp()`: it recognises the model through `fused_kind` and evaluates warp, bounds mask, image
-formation, objective and gradient in one fused GPU pass over the device-resident events
-(csrc/evk_cmax.cu).  `warp()` is still provided, with the reference's semantics, for user code that
+An objective from `event_utils_b200.contrast_max.objectives` that is handed one of the three models here
+never calls `warp()`: it recognises the model through `fused_kind` and evaluates warp, bounds mask, image
+formation, objective and gradient on the GPU over the device-resident events (csrc/evk_cmax.cu): one pass
+for linvel, two (image, then the gradient in gather form) for the rotation and xyztheta models.  `warp()` is still provided, with the reference's semantics, for user code that
 calls it directly and for the generic (non-fused) path taken by other `warp_function` subclasses.
 """
 from abc import ABC, abstractmethod
@@ -50,26 +50,52 @@ class linvel_warp(warp_function):
         return moved[0], moved[1], np.stack((-lag, nothing)), np.stack((nothing, -lag))
 
 
-class _placeholder_warp(warp_function):
-    """The reference declares these models but leaves `warp` empty (it returns None)."""
+class pure_rotation_warp(warp_function):
+    """Rotation of the image plane about a centre (cx, cy) with angular velocity omega; params = (cx, cy, omega),
+    dims = 3.  With d = t - t0, th = -omega d, c = cos th, s = sin th:
+        x' = cx + c (x - cx) - s (y - cy),       y' = cy + s (x - cx) + c (y - cy)
+        dx'/d(cx, cy, omega) = (1 - c,  s,  d (y' - cy))
+        dy'/d(cx, cy, omega) = (-s, 1 - c, -d (x' - cx))
+    The reference declares this model with an empty warp (warps.py:74-83); its README and docstring list three
+    parameters, its constructor registers dims=4, which is a slip: dims is 3 here."""
 
-    def __init__(self, name, dims):
-        super().__init__(name, dims)
+    fused_kind = "rotation"
+
+    def __init__(self):
+        super().__init__('pure_rotation_warp', 3)
 
     def warp(self, xs, ys, ts, ps, t0, params, compute_grad=False):
-        return None
+        cx, cy, omega = float(params[0]), float(params[1]), float(params[2])
+        lag = ts - t0
+        theta = -(omega * lag)
+        c, s = np.cos(theta), np.sin(theta)
+        X, Y = xs - cx, ys - cy
+        xw = cx + c * X - s * Y
+        yw = cy + s * X + c * Y
+        if not compute_grad:
+            return xw, yw, None, None
+        return xw, yw, np.stack((1 - c, s, lag * (yw - cy))), np.stack((-s, 1 - c, -(lag * (xw - cx))))
 
 
-class xyztheta_warp(_placeholder_warp):
-    """4-DoF x, y, z, rotation model (Mitrokhin et al.); an empty stub in the reference (warps.py:63-72)."""
+class xyztheta_warp(warp_function):
+    """First-order 4-DoF motion (Mitrokhin et al.): image-plane translation (vx, vy), expansion vz and in-plane
+    rotation omega about the pixel-grid origin; params = (vx, vy, vz, omega), dims = 4.  With d = t - t0:
+        x' = x - d (vx + vz x - omega y),        y' = y - d (vy + vz y + omega x)
+        dx'/d(vx, vy, vz, omega) = (-d, 0, -d x,  d y)
+        dy'/d(vx, vy, vz, omega) = (0, -d, -d y, -d x)
+    With vz = omega = 0 this is linvel_warp bit for bit.  An empty stub in the reference (warps.py:63-72)."""
+
+    fused_kind = "xyztheta"
 
     def __init__(self):
         super().__init__('xyztheta_warp', 4)
 
-
-class pure_rotation_warp(_placeholder_warp):
-    """Rotation about a centre (x, y) with angular velocity theta; an empty stub in the reference
-    (warps.py:74-83), which also registers it with dims=4."""
-
-    def __init__(self):
-        super().__init__('pure_rotation_warp', 4)
+    def warp(self, xs, ys, ts, ps, t0, params, compute_grad=False):
+        vx, vy, vz, omega = (float(v) for v in params[:4])
+        lag = ts - t0
+        xw = xs - lag * (vx + vz * xs - omega * ys)
+        yw = ys - lag * (vy + vz * ys + omega * xs)
+        if not compute_grad:
+            return xw, yw, None, None
+        nothing = np.zeros_like(lag, dtype=np.float64)
+        return xw, yw, np.stack((-lag, nothing, -(lag * xs), lag * ys)), np.stack((nothing, -lag, -(lag * ys), -(lag * xs)))

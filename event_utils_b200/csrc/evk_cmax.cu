@@ -76,9 +76,11 @@ struct CmaxArgs {
     int vec16;      // on-chip path: all four event arrays are 16-byte aligned
     float *planar;  // on-chip path: planar f32 image [npix padded to 4] the CTAs' shared-memory images are reduced into
     unsigned long long *oob;
+    double params[8];  // rotation (cx, cy, omega) / xyztheta (vx, vy, vz, omega)
 };
 
-enum { WARP_LINVEL_F64 = 0, WARP_LINVEL_F32 = 1, WARP_FLOW_F32 = 2 };
+enum { WARP_LINVEL_F64 = 0, WARP_LINVEL_F32 = 1, WARP_FLOW_F32 = 2, WARP_ROT_F64 = 3, WARP_ROT_F32 = 4, WARP_XYZT_F64 = 5, WARP_XYZT_F32 = 6 };
+__host__ __device__ constexpr bool is_model(int w) { return w >= WARP_ROT_F64; }
 
 // bilinear splat of weight w (and derivative weight a) at (xf, yf) on the canvas:
 // image.py:199-207 (IWE) and :131-135 (derivative images) with w1 = [a;0], w2 = [0;a].
@@ -216,6 +218,67 @@ __device__ __forceinline__ void splat_onchip(const CmaxArgs &A, float *acc, unsi
 // One event's four components as loaded (f64 in parity mode, f32 otherwise).
 template <int WARP> struct EvT { using type = float; };
 template <> struct EvT<WARP_LINVEL_F64> { using type = double; };
+template <> struct EvT<WARP_ROT_F64> { using type = double; };
+template <> struct EvT<WARP_XYZT_F64> { using type = double; };
+
+// ---- the rotation and xyztheta motion models (contrast_max/warps.py, include/evk.h) ----------------------
+// d = t - t_ref (f64 parity mode) or the stored t - t_last (f32 fast mode); T is the event precision.
+//   rotation  (cx, cy, omega), th = -omega d:  x' = cx + cos th (x - cx) - sin th (y - cy)
+//                                              y' = cy + sin th (x - cx) + cos th (y - cy)
+//             dx'/dp = (1 - cos th,  sin th,  d (y' - cy)),  dy'/dp = (-sin th, 1 - cos th, -d (x' - cx))
+//   xyztheta  (vx, vy, vz, omega):  x' = x - d (vx + vz x - omega y),  y' = y - d (vy + vz y + omega x)
+//             dx'/dp = (-d, 0, -d x, d y),  dy'/dp = (0, -d, -d y, -d x)
+// The operation order is the numpy order of warps.py (the library is built without FMA contraction).
+template <int WARP> struct Model {
+    static constexpr bool rot = (WARP == WARP_ROT_F64 || WARP == WARP_ROT_F32);
+    static constexpr int dims = rot ? 3 : 4;
+    using T = typename EvT<WARP>::type;
+};
+
+template <int WARP, bool JAC>
+__device__ __forceinline__ void model_warp(const CmaxArgs &A, typename Model<WARP>::T x, typename Model<WARP>::T y,
+                                           typename Model<WARP>::T d, typename Model<WARP>::T &xw, typename Model<WARP>::T &yw,
+                                           typename Model<WARP>::T *jx, typename Model<WARP>::T *jy)
+{
+    using T = typename Model<WARP>::T;
+    if constexpr (Model<WARP>::rot) {
+        const T cx = (T)A.params[0], cy = (T)A.params[1], om = (T)A.params[2];
+        const T th = -(om * d);
+        T s, c;
+        if constexpr (sizeof(T) == 8) sincos(th, &s, &c); else sincosf(th, &s, &c);
+        const T X = x - cx, Y = y - cy;
+        xw = cx + c * X - s * Y;
+        yw = cy + s * X + c * Y;
+        if (JAC) {
+            jx[0] = (T)1 - c; jx[1] = s; jx[2] = d * (yw - cy);
+            jy[0] = -s; jy[1] = (T)1 - c; jy[2] = -(d * (xw - cx));
+        }
+    } else {
+        const T vx = (T)A.params[0], vy = (T)A.params[1], vz = (T)A.params[2], om = (T)A.params[3];
+        xw = x - d * (vx + vz * x - om * y);
+        yw = y - d * (vy + vz * y + om * x);
+        if (JAC) {
+            jx[0] = -d; jx[1] = (T)0; jx[2] = -(d * x); jx[3] = d * y;
+            jy[0] = (T)0; jy[1] = -d; jy[2] = -(d * y); jy[3] = -(d * x);
+        }
+    }
+}
+
+// The polarity, time offset, warp and bounds mask of one event of a model (as the linvel branch of cmax_event).
+// Returns false when the mask drops the event.
+template <int WARP, bool JAC>
+__device__ __forceinline__ bool model_event(const CmaxArgs &A, typename Model<WARP>::T x, typename Model<WARP>::T y,
+                                            typename Model<WARP>::T t, typename Model<WARP>::T &p, typename Model<WARP>::T &xw,
+                                            typename Model<WARP>::T &yw, typename Model<WARP>::T *jx, typename Model<WARP>::T *jy)
+{
+    using T = typename Model<WARP>::T;
+    if (A.p_scale != 1.0) p = p * (T)A.p_scale;
+    if (A.abs_polarity) p = fabs(p);
+    const T d = (sizeof(T) == 8) ? t - (T)A.t_ref : t;
+    model_warp<WARP, JAC>(A, x, y, d, xw, yw, jx, jy);
+    // event_util.py:26-27: keep iff 0 < x' <= Wm and 0 < y' <= Hm (NaN compares false -> kept)
+    return !(xw <= (T)0 || xw > (T)A.Wm) && !(yw <= (T)0 || yw > (T)A.Hm);
+}
 
 template <int WARP>
 struct Event {
@@ -249,6 +312,14 @@ template <int WARP, bool GRAD, bool ONCHIP = false>
 __device__ __forceinline__ void cmax_event(const CmaxArgs &A, float *acc, const Event<WARP> &e, unsigned &oob, double cvx,
                                            double cvy, unsigned *simg = nullptr)
 {
+    if constexpr (is_model(WARP)) {
+        // pass 1 of a model: the IWE only (the gradient is cmax_model_grad_kernel's second pass)
+        typename Model<WARP>::T p = e.p, xw, yw;
+        if (!model_event<WARP, false>(A, e.x, e.y, e.t, p, xw, yw, nullptr, nullptr)) return;
+        if (ONCHIP) splat_onchip<false>(A, acc, simg, (float)xw, (float)yw, (float)p, 0.0f, true, oob);
+        else splat<false>(A, acc, (float)xw, (float)yw, (float)p, 0.0f, true, oob);
+        return;
+    }
     if (WARP == WARP_LINVEL_F64) {
         const double x = e.x, y = e.y, t = e.t;
         double p = e.p;
@@ -371,7 +442,7 @@ __global__ void __launch_bounds__(kOnchipThreads, 1) cmax_onchip_kernel(const Cm
         }
         for (int64_t j = nv * EPV + i; j < A.n; j += stride) cmax_event<WARP, GRAD, true>(A, acc, load_event<WARP>(A, j), oob, A.vx, A.vy, simg);
     } else {
-        constexpr int kB = (WARP == WARP_LINVEL_F64) ? 2 : 4;   // loads in flight per thread (64-register budget at 1024 threads)
+        constexpr int kB = sizeof(typename EvT<WARP>::type) == 8 ? 2 : 4;   // loads in flight per thread (64-register budget at 1024 threads)
         for (; i + (kB - 1) * stride < A.n; i += kB * stride) {
             Event<WARP> ev[kB];
 #pragma unroll
@@ -400,6 +471,113 @@ __global__ void __launch_bounds__(kOnchipThreads, 1) cmax_onchip_kernel(const Cm
         }
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // shared memory must outlive the engine's reads
+    }
+}
+
+// ---- pass 2 of a model: the gradient in gather form -------------------------------------------------
+// g_k = -c sum_j M[k][j] sum_pix W D_j, and the derivative images D_j are sums of per-event taps
+// (image.py:131-135 with w1 = jx p, w2 = jy p), so by adjointness
+//   sum_pix W D_j = sum_events p (jx_j Sx + jy_j Sy),   Sx = oy (W_TR - W_TL) + dy (W_BR - W_BL),
+//                                                        Sy = ox (W_BL - W_TL) + dx (W_BR - W_TR)
+// for the event's 2x2 footprint.  W (the blurred weight image of the objective, f32) sits in shared memory; the
+// events are streamed a second time and every event costs four shared-memory loads and `dims` f64 FMAs -- no
+// reductions, whatever the number of parameters.  One persistent CTA per SM.
+constexpr int kGradThreads = 512;
+
+template <int WARP>
+__device__ __forceinline__ void grad_event(const CmaxArgs &A, const float *sw, typename Model<WARP>::T x, typename Model<WARP>::T y,
+                                           typename Model<WARP>::T t, typename Model<WARP>::T p, double (&acc)[Model<WARP>::dims])
+{
+    using T = typename Model<WARP>::T;
+    constexpr int D = Model<WARP>::dims;
+    T xw, yw, jx[D], jy[D];
+    if (!model_event<WARP, true>(A, x, y, t, p, xw, yw, jx, jy)) return;
+    // the same f32 footprint as splat_taps (image.py:180-207); clipped events have zero weight, events outside
+    // the canvas were counted by pass 1 (the evaluation then fails)
+    const float xf = (float)xw, yf = (float)yw;
+    if (xf >= (float)(A.Wc - 1) || yf >= (float)(A.Hc - 1)) return;
+    const float pxf = floorf(xf), pyf = floorf(yf);
+    int x0, y0;
+    if (!trunc_checked(pxf, x0) || !trunc_checked(pyf, y0) || x0 < 0 || y0 < 0 || x0 + 1 >= A.Wc || y0 + 1 >= A.Hc) return;
+    const float dx = __fsub_rn(xf, pxf), dy = __fsub_rn(yf, pyf);
+    const float ox = __fsub_rn(1.0f, dx), oy = __fsub_rn(1.0f, dy);
+    const float *r0 = sw + y0 * A.Wc + x0, *r1 = r0 + A.Wc;
+    const double tl = r0[0], tr = r0[1], bl = r1[0], br = r1[1];
+    const double sx = (double)oy * (tr - tl) + (double)dy * (br - bl);
+    const double sy = (double)ox * (bl - tl) + (double)dx * (br - tr);
+    const double pw = (double)(float)p;   // masked_ps after the f32 cast (image.py:180)
+#pragma unroll
+    for (int j = 0; j < D; ++j) acc[j] += pw * ((double)jx[j] * sx + (double)jy[j] * sy);
+}
+
+template <int WARP>
+__global__ void __launch_bounds__(kGradThreads, 1) cmax_model_grad_kernel(const CmaxArgs A, const float *__restrict__ W, double *gk)
+{
+    using T = typename Model<WARP>::T;
+    constexpr int D = Model<WARP>::dims;
+    extern __shared__ __align__(16) float sw[];
+    const int npix = A.Hc * A.Wc;
+    for (int i = threadIdx.x; i < npix; i += kGradThreads) sw[i] = W[i];
+    __syncthreads();
+    double acc[D];
+#pragma unroll
+    for (int j = 0; j < D; ++j) acc[j] = 0.0;
+    const int64_t stride = (int64_t)gridDim.x * kGradThreads;
+    const int64_t i = (int64_t)blockIdx.x * kGradThreads + threadIdx.x;
+    const T *px = (const T *)A.x, *py = (const T *)A.y, *pt = (const T *)A.t, *pp = (const T *)A.p;
+    int64_t tail = i;
+    if (A.vec16) {
+        // 16-byte evict-first loads, two vectors of every array in flight per thread
+        constexpr int EPV = 16 / (int)sizeof(T);
+        const int64_t nv = A.n / EPV;
+        for (int64_t v = i; v < nv; v += 2 * stride) {
+            const bool two = v + stride < nv;
+            const int64_t v2 = two ? v + stride : v;
+            T ex[2][EPV], ey[2][EPV], et[2][EPV], ep[2][EPV];
+            ld_vec16(px + v * EPV, ex[0]); ld_vec16(py + v * EPV, ey[0]); ld_vec16(pt + v * EPV, et[0]); ld_vec16(pp + v * EPV, ep[0]);
+            ld_vec16(px + v2 * EPV, ex[1]); ld_vec16(py + v2 * EPV, ey[1]); ld_vec16(pt + v2 * EPV, et[1]); ld_vec16(pp + v2 * EPV, ep[1]);
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                if (h == 1 && !two) break;
+#pragma unroll
+                for (int k = 0; k < EPV; ++k) grad_event<WARP>(A, sw, ex[h][k], ey[h][k], et[h][k], ep[h][k], acc);
+            }
+        }
+        tail = nv * EPV + i;
+    }
+    for (int64_t j = tail; j < A.n; j += stride) grad_event<WARP>(A, sw, ld_stream(px + j), ld_stream(py + j), ld_stream(pt + j), ld_stream(pp + j), acc);
+    // block reduction, one global add per CTA and parameter
+    __shared__ double part[kGradThreads / 32][D];
+#pragma unroll
+    for (int j = 0; j < D; ++j) {
+        double v = acc[j];
+        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+        if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5][j] = v;
+    }
+    __syncthreads();
+    if (threadIdx.x < D) {
+        double s = 0.0;
+        for (int w = 0; w < kGradThreads / 32; ++w) s += part[w][threadIdx.x];
+        atomicAdd(gk + threadIdx.x, s);
+    }
+}
+
+// get_iwe for a model on the device (objectives.py:184-190): warped, masked positions, polarities and Jacobians
+// cast to f32 (image.py:179-183), ready for evk_image_drv_f32.  jx, jy: [dims][n].
+template <int WARP>
+__global__ void __launch_bounds__(256) cmax_model_warp_kernel(const CmaxArgs A, float *__restrict__ xo, float *__restrict__ yo,
+                                                              float *__restrict__ po, float *__restrict__ jxo, float *__restrict__ jyo)
+{
+    using T = typename Model<WARP>::T;
+    constexpr int D = Model<WARP>::dims;
+    for (int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x; i < A.n; i += (int64_t)gridDim.x * 256) {
+        T p = ((const T *)A.p)[i], xw, yw, jx[D], jy[D];
+        const T m = model_event<WARP, true>(A, ((const T *)A.x)[i], ((const T *)A.y)[i], ((const T *)A.t)[i], p, xw, yw, jx, jy) ? (T)1 : (T)0;
+        xo[i] = (float)(xw * m); yo[i] = (float)(yw * m); po[i] = (float)(p * m);
+        if (jxo) {
+#pragma unroll
+            for (int j = 0; j < D; ++j) { jxo[(int64_t)j * A.n + i] = (float)(jx[j] * m); jyo[(int64_t)j * A.n + i] = (float)(jy[j] * m); }
+        }
     }
 }
 
@@ -623,7 +801,7 @@ __global__ void __launch_bounds__(256) cmax_obj_reduce_kernel(const float *__res
         const float g = G[i];
         const double gd = (double)g;
         g1 = gd;
-        g2 = (double)(g * g);                           // np.mean(iwe*iwe): f32 product
+        g2 = kind == OBJ_VARIANCE ? gd * gd : (double)(g * g);   // variance: as cmax_blur_axis1_sums; np.mean(iwe*iwe): f32 product
         if (kind == OBJ_SOE) ge = exp(gd);              // np.exp(iwe.astype(np.double))
         if (kind == OBJ_SOSA) ga = exp(-param * gd);    // np.exp(-p*iwe.astype(np.double))
         if (kind == OBJ_ISOA) gc = (g > (float)param) ? 1.0 : 0.0;
@@ -702,6 +880,83 @@ __global__ void cmax_obj_final_kernel(int kind, const double *gsums, const unsig
     result[5] = gsums[4] / P;
     result[6] = u0;
     result[7] = u1;
+    result[8] = gsums[0] / P;
+    result[9] = gsums[2];
+    result[10] = mx;
+    result[11] = gsums[3];
+}
+
+// ---- tail of the models (any number K <= 8 of parameters): the weight image W, then f and K gradient entries ----
+constexpr int kMaxDims = 8;
+struct MixK { double m[kMaxDims][kMaxDims]; };   // scipy's blur along the length-K derivative-stack axis (objectives.py:253)
+
+// variance: W = G(2(I - mu)) = 2(G(I) - mu)  (reflect blur: self-adjoint, keeps constants)
+__global__ void __launch_bounds__(256) cmax_weight_variance_kernel(const float *__restrict__ G, const double *sums, int npix,
+                                                                   float *__restrict__ W)
+{
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= npix) return;
+    const double mu = sums[0] / (double)npix;
+    W[i] = (float)(2.0 * ((double)G[i] - mu));
+}
+
+// generic objectives: W = G(w), the axis-1 half of the blur of the per-pixel weight (cmax_blur_d_axis0_kernel is the other)
+__global__ void __launch_bounds__(256) cmax_blur_d_axis1_store_kernel(const double *__restrict__ wt, const double *__restrict__ w,
+                                                                      int Hc, int Wc, const BlurTaps taps, int do_blur, float *__restrict__ W)
+{
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= Hc * Wc) return;
+    double gw;
+    if (do_blur) {
+        const int y = i / Wc, x = i - y * Wc;
+        const double *row = wt + y * Wc;
+        gw = row[x] * taps.w[0];
+        for (int k = 1; k <= taps.r; ++k) gw += (row[reflect_idx(x - k, Wc)] + row[reflect_idx(x + k, Wc)]) * taps.w[k];
+    } else {
+        gw = w[i];
+    }
+    W[i] = (float)gw;
+}
+
+// precomputed derivative images: gk[k] = sum_pix W D_k
+__global__ void __launch_bounds__(256) cmax_dot_k_kernel(const float *__restrict__ W, const float *__restrict__ diwe, int K, int npix, double *gk)
+{
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    const double wi = i < npix ? (double)W[i] : 0.0;
+    for (int k = 0; k < K; ++k) block_add(i < npix ? wi * (double)diwe[(int64_t)k * npix + i] : 0.0, gk + k);
+}
+
+// result: the 12 slots of cmax_obj_final_kernel (variance: [5] = var); grad: K entries
+__global__ void cmax_model_final_kernel(int kind, int K, const MixK M, const double *gsums, const unsigned *gmax, const double *sums,
+                                        const double *gk, const unsigned long long *oob, int npix, int want_grad, double *result,
+                                        double *grad)
+{
+    const double P = (double)npix;
+    double f = 0.0, c = 0.0;
+    const double mx = (double)decode_ordered(*gmax);
+    const double mean_g = gsums[4] / P;
+    if (kind == OBJ_VARIANCE) { f = -(gsums[0] / P - mean_g * mean_g); c = 1.0 / P; }
+    else if (kind == OBJ_SOS) { f = -gsums[0] / P; c = 1.0 / P; }
+    else if (kind == OBJ_SOE) { f = -gsums[1] / P; c = 1.0 / P; }
+    else if (kind == OBJ_MOA) { f = -mx; c = 0.0; }
+    else if (kind == OBJ_ISOA) { f = gsums[3]; c = 1.0; }
+    else if (kind == OBJ_SOSA) { f = -gsums[2]; c = 1.0; }
+    const bool g_on = want_grad && kind != OBJ_MOA;
+    double u[kMaxDims];
+    for (int j = 0; j < kMaxDims; ++j) u[j] = (g_on && j < K) ? -c * gk[j] : 0.0;
+    for (int k = 0; k < K; ++k) {
+        double v = 0.0;
+        for (int j = 0; j < K; ++j) v += M.m[k][j] * u[j];
+        grad[k] = g_on ? v : 0.0;
+    }
+    result[0] = f;
+    result[1] = K > 0 ? grad[0] : 0.0;
+    result[2] = K > 1 ? grad[1] : 0.0;
+    result[3] = sums[0];
+    result[4] = (double)(*oob);
+    result[5] = kind == OBJ_VARIANCE ? -f : mean_g;
+    result[6] = u[0];
+    result[7] = u[1];
     result[8] = gsums[0] / P;
     result[9] = gsums[2];
     result[10] = mx;
@@ -878,6 +1133,7 @@ struct CmaxWorkspace {
     double *gsums;              // 8 doubles (generic objectives)
     unsigned *gmax;             // order-preserving encoding of max(G)
     double *sums;               // 8 doubles
+    double *gk;                 // kMaxDims doubles: sum_pix W D_k of the model tail
     unsigned long long *oob;    // 1
 };
 
@@ -896,6 +1152,7 @@ static size_t carve(void *base, int Hs, int Ws, CmaxWorkspace *ws)
     double *gsums = (double *)take(8 * sizeof(double));
     unsigned *gmax = (unsigned *)take(sizeof(unsigned));
     double *sums = (double *)take(8 * sizeof(double));
+    double *gk = (double *)take(kMaxDims * sizeof(double));
     unsigned long long *oob = (unsigned long long *)take(sizeof(unsigned long long));
     float *planar = (float *)take(((npix + 3) & ~(size_t)3) * sizeof(float));
     float *acc = (float *)take(npix * kBlockFloats * sizeof(float) * (kMaxCandidates > kMaxReplicas ? kMaxCandidates : kMaxReplicas));
@@ -908,7 +1165,7 @@ static size_t carve(void *base, int Hs, int Ws, CmaxWorkspace *ws)
     double *wt = (double *)take(npix * sizeof(double));
     if (ws) {
         ws->planar = planar; ws->acc = acc; ws->I = I; ws->D0 = D0; ws->D1 = D1; ws->tmp = tmp; ws->G = G; ws->w = w; ws->wt = wt;
-        ws->gsums = gsums; ws->gmax = gmax; ws->sums = sums; ws->oob = oob; ws->bsums = bsums; ws->btickets = btickets;
+        ws->gsums = gsums; ws->gmax = gmax; ws->sums = sums; ws->gk = gk; ws->oob = oob; ws->bsums = bsums; ws->btickets = btickets;
     }
     return off;
 }
@@ -974,6 +1231,65 @@ static int launch_tail(const CmaxWorkspace &ws, int Hc, int Wc, double sigma, un
     return EVK_OK;
 }
 
+// M[k][j] = sum_m w[|m|] [reflect(k + m, K) == j]: scipy's blur along the length-K stack axis, applied to the K
+// gradient entries (mix_coeffs is the K = 2 case); the identity without blur or with EVK_CMAX_NO_CHANNEL_MIX
+static void mix_matrix(const BlurTaps &t, int do_blur, unsigned flags, int K, MixK *M)
+{
+    memset(M, 0, sizeof(*M));
+    const bool mix = do_blur && !(flags & EVK_CMAX_NO_CHANNEL_MIX);
+    for (int k = 0; k < K; ++k) {
+        if (!mix) { M->m[k][k] = 1.0; continue; }
+        for (int m = -t.r; m <= t.r; ++m) {
+            int i = k + m;
+            const int period = 2 * K;
+            if (K == 1) i = 0;
+            else { i %= period; if (i < 0) i += period; if (i >= K) i = period - 1 - i; }
+            M->m[k][i] += t.w[m < 0 ? -m : m];
+        }
+    }
+}
+
+// The model tail on the planar IWE in ws.I (sums[0] = its sum): blur, the objective's reductions, the weight image W
+// (ws.tmp), then `pass2(W)` fills ws.gk[0..K) with sum_pix W D_k, and the final kernel writes f and the K entries.
+template <typename Pass2>
+static int model_tail(const CmaxWorkspace &ws, int Hc, int Wc, double sigma, unsigned flags, int objective, double obj_param,
+                      bool want_grad, int K, Pass2 &&pass2, double *result, double *grad, cudaStream_t st)
+{
+    if (objective < OBJ_VARIANCE || objective > OBJ_SOSA) { set_error("evk_cmax: unknown objective %d", objective); return EVK_E_ARG; }
+    const int npix = Hc * Wc;
+    BlurTaps taps{};
+    const int do_blur = sigma > 0.0;
+    if (do_blur) {
+        int rc = make_taps(sigma, &taps);
+        if (rc) return rc;
+    }
+    MixK M;
+    mix_matrix(taps, do_blur, flags, K, &M);
+    const int g = (npix + 255) / 256;
+    prof_count(do_blur ? 3 : 2);
+    if (do_blur) cmax_blur_axis0_kernel<<<g, 256, 0, st>>>(ws.I, ws.tmp, Hc, Wc, taps);
+    cmax_blur_axis1_store_kernel<<<g, 256, 0, st>>>(ws.tmp, ws.I, Hc, Wc, taps, do_blur, ws.G);
+    cmax_obj_reduce_kernel<<<g, 256, 0, st>>>(ws.G, ws.I, npix, objective, obj_param, ws.gsums, ws.gmax, ws.w);
+    const bool g_needed = want_grad && objective != OBJ_MOA;
+    if (g_needed) {
+        if (objective == OBJ_VARIANCE) {
+            prof_count(1);
+            cmax_weight_variance_kernel<<<g, 256, 0, st>>>(ws.G, ws.sums, npix, ws.tmp);
+        } else {
+            prof_count(do_blur ? 2 : 1);
+            if (do_blur) cmax_blur_d_axis0_kernel<<<g, 256, 0, st>>>(ws.w, ws.wt, Hc, Wc, taps);
+            cmax_blur_d_axis1_store_kernel<<<g, 256, 0, st>>>(ws.wt, ws.w, Hc, Wc, taps, do_blur, ws.tmp);
+        }
+        EVK_CUDA(cudaGetLastError());
+        int rc = pass2(ws.tmp);
+        if (rc) return rc;
+    }
+    prof_count(1);
+    cmax_model_final_kernel<<<1, 1, 0, st>>>(objective, K, M, ws.gsums, ws.gmax, ws.sums, ws.gk, ws.oob, npix, g_needed ? 1 : 0, result, grad);
+    EVK_CUDA(cudaGetLastError());
+    return EVK_OK;
+}
+
 // event count from which the on-chip IWE pays (EVK_CMAX_ONCHIP_MIN overrides; measured crossover, DESIGN.md section 4)
 static int64_t onchip_min_events()
 {
@@ -990,7 +1306,7 @@ static int64_t onchip_min_events()
 template <int WARP>
 static int run_cmax(CmaxArgs A, double sigma, unsigned flags, int objective, double obj_param, double *result,
                     float *iwe_out, float *diwe_out, void *workspace, size_t workspace_bytes, cudaStream_t st,
-                    float *partial_images = nullptr, unsigned long long *partial_oob = nullptr)
+                    float *partial_images = nullptr, unsigned long long *partial_oob = nullptr, double *model_grad = nullptr)
 {
     const int Hs = A.Hc - 1, Ws = A.Wc - 1;
     if (A.n < 0 || Hs < 1 || Ws < 1 || (!result && !partial_images) || !workspace) { set_error("evk_cmax: bad arguments"); return EVK_E_ARG; }
@@ -999,7 +1315,8 @@ static int run_cmax(CmaxArgs A, double sigma, unsigned flags, int objective, dou
     const size_t need = carve(workspace, Hs, Ws, &ws);
     if (workspace_bytes < need) { set_error("evk_cmax: workspace of %zu bytes required, %zu given", need, workspace_bytes); return EVK_E_WORKSPACE; }
     const int npix = A.Hc * A.Wc;
-    const bool grad = (flags & EVK_CMAX_WANT_GRAD) != 0 && WARP != WARP_FLOW_F32;
+    // a model's event pass forms the IWE only; its gradient is the second pass of model_tail
+    const bool grad = (flags & EVK_CMAX_WANT_GRAD) != 0 && WARP != WARP_FLOW_F32 && !is_model(WARP);
     A.abs_polarity = (flags & EVK_CMAX_ABS_POLARITY) ? 1 : 0;
     // replicas spread same-address serialisation in L2; small problems do not need them
     int R = (int)(A.n / (1 << 20));
@@ -1044,6 +1361,25 @@ static int run_cmax(CmaxArgs A, double sigma, unsigned flags, int objective, dou
         prof_count(1);
         if (grad) cmax_scatter_kernel<WARP, true><<<grid_for(cmax_scatter_kernel<WARP, true>, 256, A.n, 256 * 4), 256, 0, st>>>(A);
         else cmax_scatter_kernel<WARP, false><<<grid_for(cmax_scatter_kernel<WARP, false>, 256, A.n, 256 * 4), 256, 0, st>>>(A);
+    }
+    if constexpr (is_model(WARP)) {
+        prof_count(1);
+        cmax_gather_kernel<<<(npix + 255) / 256, 256, 0, st>>>(ws.acc, planar, R, A.Hc, A.Wc, ws.I, ws.D0, ws.D1, nullptr, nullptr, ws.sums);
+        auto pass2 = [&](const float *W) -> int {
+            if (A.n == 0) return EVK_OK;
+            const size_t smem = (size_t)npix * sizeof(float);
+            if (smem > (size_t)227 * 1024) { set_error("evk_cmax: a %dx%d weight image does not fit in shared memory", A.Hc, A.Wc); return EVK_E_UNSUPPORTED; }
+            EVK_CUDA(cudaFuncSetAttribute(cmax_model_grad_kernel<WARP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            const int64_t need_ctas = (A.n + kGradThreads * 8 - 1) / (kGradThreads * 8);
+            const int g = (int)(need_ctas < num_sms() ? need_ctas : num_sms());
+            ProfScope prof(st);
+            prof_count(1);
+            cmax_model_grad_kernel<WARP><<<g, kGradThreads, smem, st>>>(A, W, ws.gk);
+            EVK_CUDA(cudaGetLastError());
+            return EVK_OK;
+        };
+        return model_tail(ws, A.Hc, A.Wc, sigma, flags, objective, obj_param, (flags & EVK_CMAX_WANT_GRAD) != 0, Model<WARP>::dims,
+                          pass2, result, model_grad, st);
     }
     if (partial_images) {
         prof_count(1);
@@ -1272,6 +1608,133 @@ int evk_gaussian_blur_f32(const float *img, int H, int W, double sigma, float *o
     cmax_blur_axis1_store_kernel<<<g, 256, 0, st>>>(tmp, img, H, W, taps, do_blur, out);
     EVK_CUDA(cudaGetLastError());
     return EVK_OK;
+}
+
+static int model_dims(int model) { return model == EVK_WARP_LINVEL ? 2 : model == EVK_WARP_ROTATION ? 3 : model == EVK_WARP_XYZTHETA ? 4 : -1; }
+
+static int check_model(const char *fn, int model, const double *params, int dims)
+{
+    const int d = model_dims(model);
+    if (d < 0 || !params || dims != d) {
+        evk::set_error("%s: model %d takes %d parameters (params %p, dims %d)", fn, model, d, (const void *)params, dims);
+        return EVK_E_ARG;
+    }
+    return EVK_OK;
+}
+
+int evk_cmax_model_objective_f64(int model, const double *params, int dims, const double *x, const double *y, const double *t,
+                                 const double *p, int64_t n, double p_scale, double t_ref, int Hm, int Wm, int Hs, int Ws,
+                                 double sigma, unsigned flags, int objective, double obj_param, double *result, double *grad,
+                                 void *workspace, size_t workspace_bytes, void *stream)
+{
+    using namespace evk;
+    int rc = check_model("evk_cmax_model_objective_f64", model, params, dims);
+    if (rc) return rc;
+    if (!grad) { set_error("evk_cmax_model_objective_f64: grad is NULL"); return EVK_E_ARG; }
+    if (n > 0 && (!x || !y || !t || !p)) { set_error("evk_cmax_model_objective_f64: null event array"); return EVK_E_ARG; }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (model == EVK_WARP_LINVEL) {
+        rc = evk_cmax_linvel_objective_f64(x, y, t, p, n, p_scale, params[0], params[1], t_ref, Hm, Wm, Hs, Ws, sigma, flags, objective,
+                                           obj_param, result, nullptr, nullptr, workspace, workspace_bytes, stream);
+        if (rc) return rc;
+        EVK_CUDA(cudaMemcpyAsync(grad, result + 1, 2 * sizeof(double), cudaMemcpyDefault, st));
+        return EVK_OK;
+    }
+    CmaxArgs A{};
+    A.x = x; A.y = y; A.t = t; A.p = p; A.n = n;
+    A.t_ref = t_ref; A.p_scale = p_scale;
+    A.Hm = Hm; A.Wm = Wm; A.Hc = Hs + 1; A.Wc = Ws + 1;
+    for (int k = 0; k < dims; ++k) A.params[k] = params[k];
+    if (model == EVK_WARP_ROTATION)
+        return run_cmax<WARP_ROT_F64>(A, sigma, flags, objective, obj_param, result, nullptr, nullptr, workspace, workspace_bytes, st,
+                                      nullptr, nullptr, grad);
+    return run_cmax<WARP_XYZT_F64>(A, sigma, flags, objective, obj_param, result, nullptr, nullptr, workspace, workspace_bytes, st,
+                                   nullptr, nullptr, grad);
+}
+
+int evk_cmax_model_objective_f32(int model, const double *params, int dims, const float *x, const float *y, const float *t_rel,
+                                 const float *p, int64_t n, float p_scale, int Hm, int Wm, int Hs, int Ws, double sigma,
+                                 unsigned flags, int objective, double obj_param, double *result, double *grad, void *workspace,
+                                 size_t workspace_bytes, void *stream)
+{
+    using namespace evk;
+    int rc = check_model("evk_cmax_model_objective_f32", model, params, dims);
+    if (rc) return rc;
+    if (!grad) { set_error("evk_cmax_model_objective_f32: grad is NULL"); return EVK_E_ARG; }
+    if (n > 0 && (!x || !y || !t_rel || !p)) { set_error("evk_cmax_model_objective_f32: null event array"); return EVK_E_ARG; }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (model == EVK_WARP_LINVEL) {
+        rc = evk_cmax_linvel_objective_f32(x, y, t_rel, p, n, p_scale, (float)params[0], (float)params[1], Hm, Wm, Hs, Ws, sigma, flags,
+                                           objective, obj_param, result, nullptr, nullptr, workspace, workspace_bytes, stream);
+        if (rc) return rc;
+        EVK_CUDA(cudaMemcpyAsync(grad, result + 1, 2 * sizeof(double), cudaMemcpyDefault, st));
+        return EVK_OK;
+    }
+    CmaxArgs A{};
+    A.x = x; A.y = y; A.t = t_rel; A.p = p; A.n = n;
+    A.t_ref = 0.0; A.p_scale = p_scale;
+    A.Hm = Hm; A.Wm = Wm; A.Hc = Hs + 1; A.Wc = Ws + 1;
+    for (int k = 0; k < dims; ++k) A.params[k] = params[k];
+    if (model == EVK_WARP_ROTATION)
+        return run_cmax<WARP_ROT_F32>(A, sigma, flags, objective, obj_param, result, nullptr, nullptr, workspace, workspace_bytes, st,
+                                      nullptr, nullptr, grad);
+    return run_cmax<WARP_XYZT_F32>(A, sigma, flags, objective, obj_param, result, nullptr, nullptr, workspace, workspace_bytes, st,
+                                   nullptr, nullptr, grad);
+}
+
+int evk_cmax_model_warp_f64(int model, const double *params, int dims, const double *x, const double *y, const double *t,
+                            const double *p, int64_t n, double t_ref, int Hm, int Wm, unsigned flags, float *xw, float *yw, float *pw,
+                            float *jx, float *jy, void *stream)
+{
+    using namespace evk;
+    int rc = check_model("evk_cmax_model_warp_f64", model, params, dims);
+    if (rc) return rc;
+    if (model == EVK_WARP_LINVEL) { set_error("evk_cmax_model_warp_f64: linvel images come from evk_cmax_linvel_objective_f64"); return EVK_E_ARG; }
+    if (n < 0 || (n > 0 && (!x || !y || !t || !p || !xw || !yw || !pw)) || (!jx != !jy)) {
+        set_error("evk_cmax_model_warp_f64: bad arguments");
+        return EVK_E_ARG;
+    }
+    if (n == 0) return EVK_OK;
+    CmaxArgs A{};
+    A.x = x; A.y = y; A.t = t; A.p = p; A.n = n;
+    A.t_ref = t_ref; A.p_scale = 1.0; A.abs_polarity = (flags & EVK_CMAX_ABS_POLARITY) ? 1 : 0;
+    A.Hm = Hm; A.Wm = Wm;
+    for (int k = 0; k < dims; ++k) A.params[k] = params[k];
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    prof_count(1);
+    if (model == EVK_WARP_ROTATION)
+        cmax_model_warp_kernel<WARP_ROT_F64><<<grid_simple(n, 256 * 4), 256, 0, st>>>(A, xw, yw, pw, jx, jy);
+    else
+        cmax_model_warp_kernel<WARP_XYZT_F64><<<grid_simple(n, 256 * 4), 256, 0, st>>>(A, xw, yw, pw, jx, jy);
+    EVK_CUDA(cudaGetLastError());
+    return EVK_OK;
+}
+
+int evk_iwe_objective_k_f32(const float *iwe, const float *diwe, int K, int Hc, int Wc, double sigma, unsigned flags, int objective,
+                            double obj_param, double *result, double *grad, void *workspace, size_t workspace_bytes, void *stream)
+{
+    using namespace evk;
+    if (!iwe || !result || !workspace || Hc < 2 || Wc < 2 || K < 0 || K > kMaxDims || (K > 0 && (!diwe || !grad))) {
+        set_error("evk_iwe_objective_k_f32: bad arguments (0 <= K <= %d)", kMaxDims);
+        return EVK_E_ARG;
+    }
+    if (((uintptr_t)workspace & 255) != 0) { set_error("evk_iwe_objective_k_f32: workspace must be 256-byte aligned"); return EVK_E_ARG; }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    CmaxWorkspace ws;
+    const size_t need = carve(workspace, Hc - 1, Wc - 1, &ws);
+    if (workspace_bytes < need) { set_error("evk_iwe_objective_k_f32: workspace of %zu bytes required", need); return EVK_E_WORKSPACE; }
+    const int npix = Hc * Wc;
+    EVK_CUDA(cudaMemsetAsync(ws.gsums, 0, (size_t)((char *)(ws.oob + 1) - (char *)ws.gsums), st));
+    prof_count(1);
+    cmax_planar_kernel<<<(npix + 255) / 256, 256, 0, st>>>(iwe, nullptr, npix, ws.I, ws.D0, ws.D1, ws.sums);
+    auto pass2 = [&](const float *W) -> int {
+        prof_count(1);
+        cmax_dot_k_kernel<<<(npix + 255) / 256, 256, 0, st>>>(W, diwe, K, npix, ws.gk);
+        EVK_CUDA(cudaGetLastError());
+        return EVK_OK;
+    };
+    return model_tail(ws, Hc, Wc, sigma, flags, objective, obj_param, (flags & EVK_CMAX_WANT_GRAD) != 0 && K > 0, K, pass2, result,
+                      grad, st);
 }
 
 int evk_cmax_linvel_objective_batch_f64(const double *x, const double *y, const double *t, const double *p, int64_t n,

@@ -298,6 +298,60 @@ int evk_iwe_objective_f32(const float *iwe, const float *diwe, int Hc, int Wc, d
                           unsigned flags, int objective, double obj_param, double *result,
                           void *workspace, size_t workspace_bytes, void *stream);
 
+/* ---------------------------------------------------------------------------------------------
+ * Contrast maximisation for every motion model of lib/contrast_max/warps.py (README: linvel_warp,
+ * xyztheta_warp, pure_rotation_warp).  The reference leaves the last two empty (warps.py:63-83); this
+ * library defines them (contrast_max/warps.py).  d = t - t_ref, events transported back to t_ref:
+ *   EVK_WARP_LINVEL     (vx, vy)            warps.py:51-61; dispatches to evk_cmax_linvel_objective_* (same bits)
+ *   EVK_WARP_ROTATION   (cx, cy, omega)     th = -omega d:  x' = cx + cos th (x-cx) - sin th (y-cy),
+ *                                                           y' = cy + sin th (x-cx) + cos th (y-cy)
+ *                       dx'/dp = (1 - cos th, sin th, d (y'-cy)),  dy'/dp = (-sin th, 1 - cos th, -d (x'-cx))
+ *   EVK_WARP_XYZTHETA   (vx, vy, vz, omega) x' = x - d (vx + vz x - omega y),  y' = y - d (vy + vz y + omega x)
+ *                       dx'/dp = (-d, 0, -d x, d y),  dy'/dp = (0, -d, -d y, -d x)
+ * Everything after the warp is get_iwe + the objective as for linvel (objectives.py:184-192, image.py:179-217,
+ * objectives.py:231-264 and :266-523): f64 warp and bounds mask, f32 cast, the fixed (Hs+1)x(Ws+1) canvas.
+ * The derivative images have `dims` channels (image.py:210 allocates 2; interpolate_to_derivative_img,
+ * image.py:131-135, already loops over all of them), and scipy's 3-D blur of the (dims,H,W) stack mixes the
+ * gradient entries by M[k][j] = sum_m w[|m|] [reflect(k+m, dims) == j] (objectives.py:253;
+ * EVK_CMAX_NO_CHANNEL_MIX: identity).
+ * Rotation and xyztheta run two passes over the events: pass 1 forms the IWE (the linvel event-pass kernels);
+ * pass 2 is the gradient in GATHER form, g_k = -c sum_j M[k][j] sum_events p (jx_j Sx + jy_j Sy), with W the
+ * blurred weight image of the objective held in shared memory and Sx, Sy the x / y differences of W over the
+ * event's 2x2 footprint -- the same cost for any number of parameters.
+ *   params : `dims` doubles in HOST memory; dims must be the model's (2, 3, 4)
+ *   result : the 12 doubles of evk_cmax_linvel_objective_* ([1],[2] = grad[0], grad[1]); grad: `dims` doubles,
+ *            device-addressable (device or pinned host memory)
+ *   _f32   : fast mode, t_rel = t - t_ref already subtracted, as evk_cmax_linvel_objective_f32
+ * workspace: evk_cmax_workspace_bytes(Hs,Ws) bytes, 256-byte aligned.
+ * --------------------------------------------------------------------------------------------- */
+#define EVK_WARP_LINVEL 0
+#define EVK_WARP_ROTATION 1
+#define EVK_WARP_XYZTHETA 2
+int evk_cmax_model_objective_f64(int model, const double *params, int dims, const double *x,
+                                 const double *y, const double *t, const double *p, int64_t n,
+                                 double p_scale, double t_ref, int Hm, int Wm, int Hs, int Ws,
+                                 double sigma, unsigned flags, int objective, double obj_param,
+                                 double *result, double *grad, void *workspace,
+                                 size_t workspace_bytes, void *stream);
+int evk_cmax_model_objective_f32(int model, const double *params, int dims, const float *x,
+                                 const float *y, const float *t_rel, const float *p, int64_t n,
+                                 float p_scale, int Hm, int Wm, int Hs, int Ws, double sigma,
+                                 unsigned flags, int objective, double obj_param, double *result,
+                                 double *grad, void *workspace, size_t workspace_bytes, void *stream);
+/* get_iwe's warp and mask for a model on the device (objectives.py:184-190): xw, yw, pw = x', y', p times the
+ * bounds mask, jx, jy = [dims][n] Jacobians times the mask (may both be NULL), all cast to f32 as
+ * events_to_image_drv does (image.py:179-183) -- the inputs of evk_image_drv_f32.  Rotation / xyztheta only;
+ * EVK_CMAX_ABS_POLARITY: p <- |p|. */
+int evk_cmax_model_warp_f64(int model, const double *params, int dims, const double *x, const double *y,
+                            const double *t, const double *p, int64_t n, double t_ref, int Hm, int Wm,
+                            unsigned flags, float *xw, float *yw, float *pw, float *jx, float *jy,
+                            void *stream);
+/* The precomputed-image form with K <= 8 derivative channels (diwe: [K][Hc][Wc]) and K gradient entries
+ * (grad, device-addressable); result as above.  For any warp, including user-defined ones. */
+int evk_iwe_objective_k_f32(const float *iwe, const float *diwe, int K, int Hc, int Wc, double sigma,
+                            unsigned flags, int objective, double obj_param, double *result,
+                            double *grad, void *workspace, size_t workspace_bytes, void *stream);
+
 /* scipy.ndimage.gaussian_filter(img, sigma) for a 2-D f32 image (truncate=4, mode='reflect', f64 line
  * accumulation, f32 store after each axis) -- the blur every objective applies (objectives.py:233 ...).
  * tmp: H*W floats of scratch; out may not alias img. */
